@@ -101,7 +101,15 @@ def parse():
     ap.add_argument("--zero1", action="store_true", help="shard the fp32 optimizer state over the ranks (ZeRO-1)")
     ap.add_argument("--lean", action="store_true",
                     help="profiling aid (ncu launch lists): skip the e2e and roofline passes; the line is NOT a bench value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32; "
+                         "large arrays as a fixed, seeded sample) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ivb200":
+        ap.error("--dump-outputs writes the outputs of the ivb200 arm")
+    return args
 
 
 def host_cores():
@@ -204,6 +212,35 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_MAX_ELEMS = 1 << 22          # per array: 16 MB of float32; at most 3 arrays per task stay under 64 MB in all
+PARAM_SAMPLE = 4096               # elements sampled from every parameter
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: each tensor as out_dir/<name>.npy in float32.  A tensor of more than DUMP_MAX_ELEMS elements is
+    replaced by the elements at DUMP_MAX_ELEMS fixed, seeded positions (the same positions in every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for i, (name, t) in enumerate(arrays.items()):
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(i)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
+def param_sample(model):
+    """PARAM_SAMPLE elements at fixed, seeded positions of every parameter (in named_parameters() order), concatenated."""
+    import torch
+    g = torch.Generator().manual_seed(0)
+    parts = []
+    for _, p in model.named_parameters():
+        idx = torch.randint(p.numel(), (min(p.numel(), PARAM_SAMPLE),), generator=g).sort().values
+        parts.append(p.detach().reshape(-1)[idx.to(p.device)].float())
+    return torch.cat(parts)
+
+
 def make_mask(B, T, L, keep, seed):
     """Attention-style mask of the recipe with uniform importance: per frame keep 52 of 256 patches
     (engine_for_pretraining.py:105-116), cls always visible.  bool [B, 1+T*L], True = masked."""
@@ -278,6 +315,8 @@ def run_attn(args):
         flush.zero_()
         e0.record(); step(); e1.record()
     sync()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"out": out, "lse": lse, "dqkv": dqkv})
     ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = ll.launch_count()
     # end to end: the projection buffer comes from pinned host memory, one gradient element is read back
@@ -343,7 +382,8 @@ def attention_roofline(attn, nprof, ms_step, peak=None):
 def measure(args, world, local, step, dev_inputs, host_inputs, engine):
     """Warm up, capture the step into one CUDA graph, then time: (1) K steps on device-resident inputs, (2) K steps
     fed from pinned HOST buffers with the loss read back every step (e2e), (3) a few eager steps with CUDA events
-    around every GEMM launch (roofline).  Barrier + synchronize on both sides, max over ranks."""
+    around every GEMM launch (roofline).  Barrier + synchronize on both sides, max over ranks.  With --dump-outputs,
+    the loss of the last step of (1) and a sample of the parameters it left are written before (2) changes them."""
     import torch
     import torch.distributed as dist
     from internvideo_b200 import lowlevel as ll
@@ -386,6 +426,8 @@ def measure(args, world, local, step, dev_inputs, host_inputs, engine):
     e1.record(); sync()
     if args.lean:
         torch.cuda.profiler.stop()
+    if args.dump_outputs and int(os.environ.get("RANK", 0)) == 0:
+        write_outputs(args.dump_outputs, {"loss": loss, "params_sample": param_sample(engine.model)})
     ms = e0.elapsed_time(e1)
     launches = ll.launch_count() if graphed is None else launches_per_step * args.steps
     # -------- end-to-end timing through the public API with HOST buffers (e2e)

@@ -21,6 +21,9 @@ Fixtures
                      rank, loss, and the per-rank input gradients (local-slice backward semantics).
   pixel_target.npz   IV1 VideoMAE target construction: the reference's own statements
                      (engine_for_pretraining.py:66-98) exec'd on a seeded clip.
+  ref_checks.npz     small results of reference functions and modules that the CPU tests check host code against:
+                     mask generators, position tables and interpolation, a reference-built model's attributes, an
+                     InternVideo2-S forward on seeded weights (sampled), stage-2 criterions, recall@k, IV1 init digests.
 """
 from __future__ import annotations
 
@@ -616,12 +619,224 @@ def make_iv1_videomae():
     print("iv1_videomae: out", tuple(out.shape), "loss", float(loss), "enc", tuple(blob["enc_out"].shape))
 
 
+def _json(obj):
+    return np.frombuffer(json.dumps(obj).encode(), dtype=np.uint8)
+
+
+def seeded_state(layout, seed):
+    """Seeded weights for a state_dict layout [(key, shape), ...] that is too large to store: LayerScale around 0.1,
+    norm weights around 1, small biases, every other tensor N(0, 0.02).  Regenerated wherever the fixture is used."""
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for k, shape in layout:
+        t = torch.randn(tuple(shape), generator=g)
+        if k.endswith("gamma"):
+            t = 0.1 * (1 + 0.3 * t)
+        elif "norm" in k and k.endswith("weight"):
+            t = 1 + 0.1 * t
+        elif k.endswith("bias"):
+            t = 0.05 * t
+        else:
+            t = 0.02 * t
+        sd[k] = t
+    return sd
+
+
+def describe_module(model, exact_max_numel=4096):
+    """What code that reads hyper-parameters off a built module can see, without the module's source: per submodule its
+    kind (list or not), its plain attributes, and its parameters and buffers (None where registered as None).  Tensors of
+    up to `exact_max_numel` elements are stored exactly, larger ones only as a (key, shape) layout for seeded_state(layout, 0)."""
+    def plain(v):
+        if v is None or isinstance(v, (bool, int, float, str)):
+            return True
+        return isinstance(v, (list, tuple)) and all(plain(x) for x in v)
+
+    mods, exact, layout = [], {}, []
+    for name, m in model.named_modules():
+        tensors = []
+        for kind, store in (("p", m._parameters), ("b", m._buffers)):
+            for k, t in store.items():
+                full = f"{name}.{k}" if name else k
+                persistent = kind == "p" or k not in m._non_persistent_buffers_set
+                tensors.append([kind, k, None if t is None else list(t.shape), persistent])
+                if t is None:
+                    continue
+                if t.numel() <= exact_max_numel:
+                    exact[full] = t.detach().numpy().copy()
+                else:
+                    layout.append((full, list(t.shape)))
+        mods.append(dict(name=name, is_list=isinstance(m, (torch.nn.ModuleList, torch.nn.Sequential)),
+                         attrs={k: v for k, v in vars(m).items() if not k.startswith("_") and plain(v)}, tensors=tensors))
+    return dict(modules=mods, seeded_layout=layout), exact
+
+
+def sample_flat(t, n, seed):
+    """A fixed, seeded sample of n elements of t (flattened), in index order."""
+    flat = t.detach().reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    return flat[idx]
+
+
+SDIMS_CFG = dict(embed_dim=384, depth=12, num_heads=6, mlp_ratio=4, num_frames=4, drop_path_rate=0.0,
+                 clip_return_layer=1, mae_return_layer=1, attn_pool_num_heads=16, init_values=0.1)
+SDIMS_SEED = 2025
+FROM_REF_CFG = dict(embed_dim=176, depth=3, num_heads=2, mlp_ratio=48 / 11, num_frames=2, img_size=56, patch_size=14,
+                    drop_path_rate=0.3, attn_pool_num_heads=2, clip_embed_dim=64, clip_teacher_embed_dim=96,
+                    clip_teacher_final_dim=64, mae_teacher_embed_dim=176, clip_return_layer=2, mae_return_layer=2,
+                    clip_student_return_interval=1, init_values=0.08)
+SEP_POS_CFG = dict(sep_pos_embed=True, embed_dim=64, depth=1, num_heads=2, num_frames=2, img_size=28,
+                   clip_teacher_embed_dim=32, clip_teacher_final_dim=16, mae_teacher_embed_dim=64, attn_pool_num_heads=2,
+                   clip_embed_dim=16)
+IV1_INIT_CFG = dict(img_size=32, patch_size=16, encoder_embed_dim=128, encoder_depth=1, encoder_num_heads=2,
+                    decoder_num_classes=1536, decoder_embed_dim=64, decoder_depth=1, decoder_num_heads=1, qkv_bias=True,
+                    init_values=0.1)
+
+
+def sdims_inputs():
+    """Input clips and mask of the InternVideo2-S restatement check (BASELINE cfg-1: 2 clips x 4 frames x 224^2)."""
+    g = torch.Generator().manual_seed(SDIMS_SEED + 1)
+    x = torch.randn(2, 3, 4, 224, 224, generator=g)
+    g = torch.Generator().manual_seed(3)
+    mask = torch.ones(2, 1 + 4 * 256, dtype=torch.bool)
+    mask[:, 0] = False
+    for b in range(2):
+        for t in range(4):
+            mask[b, 1 + t * 256 + torch.randperm(256, generator=g)[:52]] = False
+    return x, mask
+
+
+def make_ref_checks():
+    """Small results of the unmodified reference that the CPU tests compare the project's host code against, one entry
+    group per check (tests/test_masking_cpu.py, test_modules_cpu.py, test_oracle_cpu.py, test_stage2_cpu.py,
+    test_videomae_v1_cpu.py).  Inputs are regenerated from the same seeds in the tests."""
+    import contextlib, hashlib, importlib, io, types
+    import importlib.util
+    blob = {}
+
+    def load(path, name):
+        spec = importlib.util.spec_from_file_location(name, path)
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+        return mod
+
+    # batch mask generators (multi_modality/models/mask.py) under fixed numpy seeds
+    mm_mask = load(os.path.join(ref_shim.IV2_MM, "models", "mask.py"), "_ivref_mm_mask")
+    for i, (size, ratio, B) in enumerate((((8, 16, 16), 0.8, 4), ((1, 14, 14), 0.5, 3), ((4, 16, 16), 0.9, 2))):
+        np.random.seed(11); blob[f"mask/tube{i}"] = mm_mask.TubeMaskingGenerator(size, ratio, B, device="cpu").numpy()
+        np.random.seed(12); blob[f"mask/random{i}"] = mm_mask.RandomMaskingGenerator(size, ratio, B, device="cpu").numpy()
+    # per-clip mask generators (single_modality/datasets/masking_generator.py)
+    sm_mask = load(os.path.join(ref_shim.IV2_SM, "datasets", "masking_generator.py"), "_ivref_sm_maskgen")
+    for i, (size, ratio) in enumerate((((8, 14, 14), 0.9), ((4, 16, 16), 0.8))):
+        np.random.seed(5); blob[f"clipmask/tube{i}"] = np.stack([sm_mask.TubeMaskingGenerator(size, ratio)() for _ in range(3)])
+        blob[f"clipmask/tube_repr{i}"] = _json(repr(sm_mask.TubeMaskingGenerator(size, ratio)))
+        np.random.seed(6); blob[f"clipmask/random{i}"] = np.stack([sm_mask.RandomMaskingGenerator(size, ratio)() for _ in range(3)])
+
+    # 3-D sin-cos table, separable position tables and pos-embed interpolation
+    sm = ref_shim.import_single_modality()
+    blob["pos/sincos_64_4_2_cls"] = np.asarray(sm.get_3d_sincos_pos_embed(64, 4, 2, cls_token=True))
+    ref = ref_shim.build_reference_model(**SEP_POS_CFG)
+    rs = ref.state_dict()
+    blob["seppos/keys"] = _json(list(rs))
+    for k, t in rs.items():
+        if "pos_embed" in k:
+            blob["seppos/" + k] = t.numpy()
+    ref_shim.import_clip_vision()
+    pe = importlib.import_module("_ivref_mm_backbone.pos_embed")
+    from internvideo_b200.clip_modules import InternVideo2
+    tower = InternVideo2(embed_dim=64, depth=1, num_heads=2, num_frames=8, img_size=112, attn_pool_num_heads=2,
+                         clip_embed_dim=16, use_flash_attn=False, use_fused_rmsnorm=False, use_fused_mlp=False)
+    ck = {"vision_encoder.pos_embed": torch.randn(1, 1 + 4 * 16, 64, generator=torch.Generator().manual_seed(0))}
+    with contextlib.redirect_stdout(io.StringIO()):
+        pe.interpolate_pos_embed(ck, tower, orig_t_size=4)
+    out = ck["vision_encoder.pos_embed"]
+    blob["interp/shape"] = np.asarray(out.shape, dtype=np.int64)
+    blob["interp/sample"], blob["interp/norm"] = sample_flat(out, 4096, 99).numpy(), np.float64(out.double().norm())
+
+    # a reference-built PretrainInternVideo2 as patch.from_reference sees it
+    desc, exact = describe_module(ref_shim.build_reference_model(**FROM_REF_CFG).train())
+    blob["fromref/desc"] = _json(desc)
+    for k, t in exact.items():
+        blob["fromref/t/" + k] = t
+
+    # InternVideo2-S student forward (naive path, fp32) on seeded weights: a seeded sample of every output + its norm
+    model = ref_shim.build_reference_model(**SDIMS_CFG).eval()
+    layout = [(k, list(t.shape)) for k, t in model.state_dict().items()]
+    model.load_state_dict(seeded_state(layout, SDIMS_SEED), strict=True)
+    x, mask = sdims_inputs()
+    with torch.no_grad():
+        outs = model(x, mask)
+    blob["sdims/layout"] = _json(layout)
+    for i, o in enumerate(outs):
+        blob[f"sdims/shape{i}"] = np.asarray(o.shape, dtype=np.int64)
+        blob[f"sdims/sample{i}"] = sample_flat(o, 4096, 100 + i).numpy()
+        blob[f"sdims/norm{i}"] = np.float64(o.double().norm())
+
+    # stage-2 criterions: the triplets vtm_loss hands its fusion encoder, uta_loss, get_sim
+    crit, _ = ref_shim.import_criterions()
+    for hard in (True, False):
+        g = torch.Generator().manual_seed(3)
+        B, Lv, Lt, C = 12, 5, 4, 16
+        vis = torch.randn(B, Lv, C, generator=g); txt = torch.randn(B, Lt, C, generator=g)
+        vp = torch.randn(B, C, generator=g); tp = torch.randn(B, C, generator=g)
+        atts = (torch.rand(B, Lt, generator=g) > 0.3).long()
+        idx = torch.arange(B); idx[7] = 2
+        seen = {}
+
+        def encoder(encoder_embeds, attention_mask, encoder_hidden_states, encoder_attention_mask, return_dict, mode):
+            seen.update(text=encoder_embeds, atts=attention_mask, vision=encoder_hidden_states)
+            return types.SimpleNamespace(last_hidden_state=encoder_embeds)
+
+        head = torch.nn.Linear(C, 2)
+        torch.manual_seed(77)
+        crit.VTC_VTM_Loss(hard).vtm_loss(encoder, head, 0.07, vis, txt, vp, tp, atts, idx)
+        for k, t in seen.items():
+            blob[f"vtm/{int(hard)}/{k}"] = t.detach().numpy()
+    g = torch.Generator().manual_seed(9)
+    s = torch.randn(2, 3, 7, 20, generator=g); c = torch.randn(2, 3, 7, 20, generator=g)
+    for norm in ("l2", "none"):
+        for kind in ("l2", "mse", "smooth_l1"):
+            blob[f"uta/{norm}/{kind}"] = crit.UTA_Loss(norm, kind).uta_loss(s, c).numpy()
+    v = torch.randn(6, 16, generator=g); t = torch.randn(5, 16, generator=g)
+    blob["sim/2d/v2t"], blob["sim/2d/t2v"] = (a.numpy() for a in crit.get_sim(v, t, 0.07))
+    v3 = torch.randn(6, 4, 16, generator=g)
+    for agg in ("mean", "max"):
+        blob[f"sim/v3/{agg}/v2t"], blob[f"sim/v3/{agg}/t2v"] = (a.numpy() for a in crit.get_sim(v3, t, 0.07, agg))
+    t3 = torch.randn(5, 3, 16, generator=g)
+    for agg in ("mean", "max"):
+        blob[f"sim/t3/{agg}/v2t"], blob[f"sim/t3/{agg}/t2v"] = (a.numpy() for a in crit.get_sim(v, t3, 0.07, agg))
+    # recall@k of tasks_clip/retrieval_utils.py::itm_eval (the function alone: its module imports the whole project)
+    path = os.path.join(ref_shim.IV2_MM, "tasks_clip", "retrieval_utils.py")
+    src = open(path).read()
+    start = src.index("def itm_eval(")
+    ns = {"np": np}
+    exec(compile(src[start:src.index("\n\n\n", start)] if "\n\n\n" in src[start:] else src[start:], path, "exec"), ns)
+    rg = np.random.default_rng(4)
+    s = rg.standard_normal((9, 13)).astype(np.float32)
+    txt2img = [int(x) for x in rg.integers(0, 9, 13)]
+    img2txt = [[j for j in range(13) if txt2img[j] == i] or [0] for i in range(9)]
+    blob["itm_eval"] = _json({k: float(v) for k, v in ns["itm_eval"](s, s.T.copy(), txt2img, img2txt).items()})
+
+    # InternVideo1 VideoMAE: fixed sinusoid tables, key order, and a digest of every initial tensor under one seed
+    iv1 = ref_shim.import_iv1_videomae()
+    torch.manual_seed(3)
+    net = iv1.PretrainVisionTransformer(**IV1_INIT_CFG)
+    blob["iv1/pos_embed"] = net.pos_embed.numpy()
+    blob["iv1/encoder_pos_embed"] = net.encoder.pos_embed.numpy()
+    blob["iv1/init_sha256"] = _json([[k, list(t.shape), hashlib.sha256(t.contiguous().numpy().tobytes()).hexdigest()]
+                                     for k, t in net.state_dict().items()])
+
+    np.savez_compressed(GOLD / "ref_checks.npz", **blob)
+    print("ref_checks:", len(blob), "entries,", os.path.getsize(GOLD / "ref_checks.npz"), "bytes")
+
+
 if __name__ == "__main__":
     assert ref_shim.available(), "reference not mounted"
     GOLD.mkdir(parents=True, exist_ok=True)
-    which = sys.argv[1:] or ["pretrain_tiny", "pretrain_d88", "pretrain_dp", "block_cfg2", "clip_small", "teachers", "vtc", "pixel_target", "stage2", "iv1_videomae"]
+    which = sys.argv[1:] or ["pretrain_tiny", "pretrain_d88", "pretrain_dp", "block_cfg2", "clip_small", "teachers", "vtc",
+                             "pixel_target", "stage2", "iv1_videomae", "ref_checks"]
     makers = {"pretrain_tiny": make_pretrain_tiny, "pretrain_d88": make_pretrain_d88, "vtc": make_vtc,
               "pixel_target": make_pixel_target, "pretrain_dp": make_pretrain_dp, "block_cfg2": make_block_cfg2,
-              "clip_small": make_clip_small, "teachers": make_teachers, "stage2": make_stage2, "iv1_videomae": make_iv1_videomae}
+              "clip_small": make_clip_small, "teachers": make_teachers, "stage2": make_stage2, "iv1_videomae": make_iv1_videomae,
+              "ref_checks": make_ref_checks}
     for w in which:      # e.g. `python oracle/make_golden.py pretrain_d88` regenerates one fixture only
         makers[w]()
